@@ -28,6 +28,11 @@ sides, max over ranks.
   python bench.py --gpus 1 --steps 5 --warmup 3
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 ... bench.py --gpus N ...
   python bench.py --impl reference      # the CPU restatement of the reference path on the host cores
+  python bench.py --dump-outputs bench_outputs   # + what the last timed step computed, as .npy files
+
+`--dump-outputs DIR` writes, after the timed steps, the arrays the last timed step handed its caller on rank 0, as float64
+DIR/<name>.npy: whole when small, else at a fixed sample of rows (seed 0, `rows.npy`), at most DUMP_BYTES in all.  The
+inputs are generated from fixed seeds, so two builds of the project can be compared output for output.
 
 The CPU oracle (oracle/) is used here only for `cpu_baseline`, `--impl reference` and the post-run verification; the
 measured GPU path never touches it.
@@ -49,8 +54,10 @@ import numpy as np
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark leaves the source tree as it found it
 
 METRIC = "geometries/s"
+DUMP_BYTES = 64_000_000  # --dump-outputs writes at most this many bytes
 MIN_LOAD_S = 0.6  # seconds of warm-up load before the timed region (so that the nvidia-smi clock sampler has samples under load)
 COORD_BYTES = 16  # one f64 xy pair: the algorithmic bytes per coordinate (SURVEY.md §8d)
 
@@ -85,6 +92,26 @@ def recorded_traffic(name):
 
 def all_cpus():
     return sorted(os.sched_getaffinity(0)) if hasattr(os, "sched_getaffinity") else list(range(os.cpu_count() or 1))
+
+
+def sample_rows(n, k, device):
+    """row numbers of a --dump-outputs sample: all n rows when n <= k, else k distinct rows drawn with seed 0, ascending"""
+    import torch
+
+    if n <= k:
+        return torch.arange(n, device=device)
+    rows = np.sort(np.random.default_rng(0).choice(n, size=k, replace=False))
+    return torch.from_numpy(rows).to(device)
+
+
+def write_outputs(directory, arrays):
+    """--dump-outputs: one float64 DIR/<name>.npy per array"""
+    arrays = {k: np.ascontiguousarray(v.cpu().numpy() if hasattr(v, "cpu") else v, dtype=np.float64) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_BYTES, f"--dump-outputs: {total} bytes exceed the {DUMP_BYTES}-byte budget"
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
 
 
 class ClockSampler:
@@ -296,6 +323,17 @@ class JoinWorkload:
     def workload_text(self):
         return f"{self.n} random points per GPU .contains() x {self.n_polys} {self.nvert}-vertex polygons ({self.baseline})"
 
+    def outputs(self):
+        """the id column (first containing polygon, -1 for none) at sampled rows, and every per-polygon hit count.  With
+        the column gathered (c4 on several GPUs) rank 0 holds every rank's rows: rank r's rows follow as r * n + row."""
+        import torch
+
+        segments = self.gathered or [self.ids]
+        n = self.n
+        rows = sample_rows(n * len(segments), 2_000_000, self.env.dev)
+        ids = torch.cat([seg[rows[(rows >= r * n) & (rows < (r + 1) * n)] - r * n] for r, seg in enumerate(segments)])
+        return {"rows": rows, "ids": ids, "counts": self.last_counts}
+
     # --- correctness, outside the timed region ----------------------------------------------------------------
     def verify(self):
         import torch
@@ -446,6 +484,14 @@ class PairsWorkload:
 
     def workload_text(self):
         return f"{self.total} LineString pairs, {self.K} coordinates each, euclidean_distance + intersects (BASELINE configs[2]; SURVEY.md config 3 generator)"
+
+    def outputs(self):
+        """distance and intersects (0 / 1) of sampled pairs of this rank's row range"""
+        import torch
+
+        rows = sample_rows(self.n, 2_000_000, self.env.dev)
+        bits = self.bits[rows // 8].to(torch.int64)
+        return {"rows": rows, "distance": self.dist_out[rows], "intersects": (bits >> (rows % 8)) & 1}
 
     def verify(self):
         from geopolars_b200 import GeoArrowArray, synth
@@ -609,19 +655,50 @@ class HullWorkload:
     def workload_text(self):
         return f"{self.total} polygons x {self.NV + 1} coordinates, convex_hull + affine_transform (BASELINE configs[4]; SURVEY.md config 5 generator)"
 
-    def verify(self):
+    def hull_rings(self):
+        """the last step's hull column as device tensors: ring offsets (g + 1) and coordinates"""
         import torch
 
         from geopolars_b200 import engine as E
-        from oracle import oracle as og
 
         e = self.env
-        m, nv = min(self.g, self.args.verify_rows), self.NV
-        hv = self.hull.view()
         hro = torch.empty(self.g + 1, dtype=torch.int64, device=e.dev)
-        hxy = torch.empty((hv.n_coords, 2), dtype=torch.float64, device=e.dev)
+        hxy = torch.empty((self.hull.view().n_coords, 2), dtype=torch.float64, device=e.dev)
         E.check(e.ctx.lib.gpl_array_copy_out(e.ctx._h, self.hull._h, C.c_void_p(hxy.data_ptr()), None, None, C.c_void_p(hro.data_ptr()), None, E.GPL_DEVICE))
         e.stream.synchronize()
+        return hro, hxy
+
+    def moved_coords(self):
+        """the last step's affine_transform output as a (coordinates, 2) device tensor"""
+        import torch
+
+        from geopolars_b200 import engine as E
+
+        e = self.env
+        mv = torch.empty((self.nc, 2), dtype=torch.float64, device=e.dev)
+        E.check(e.ctx.lib.gpl_array_copy_out(e.ctx._h, self.moved._h, C.c_void_p(mv.data_ptr()), None, None, None, None, E.GPL_DEVICE))
+        e.stream.synchronize()
+        return mv
+
+    def outputs(self):
+        """hull rings (coordinate counts and concatenated coordinates) and transformed coordinates of sampled polygons"""
+        import torch
+
+        rows = sample_rows(self.g, 4096, self.env.dev)
+        hro, hxy = self.hull_rings()
+        start = hro[rows]
+        lens = hro[rows + 1] - start
+        first = torch.cumsum(lens, 0) - lens  # where each sampled ring starts in the concatenation
+        at = torch.repeat_interleave(start - first, lens) + torch.arange(int(lens.sum()), device=self.env.dev)
+        moved = self.moved_coords().view(self.g, self.NV + 1, 2)[rows].reshape(-1, 2)
+        return {"rows": rows, "hull_ring_len": lens, "hull_xy": hxy[at], "affine_xy": moved}
+
+    def verify(self):
+        from oracle import oracle as og
+
+        m, nv = min(self.g, self.args.verify_rows), self.NV
+        hv = self.hull.view()
+        hro, hxy = self.hull_rings()
         xy = self.xy[: m * (nv + 1)].cpu().numpy()  # the device generator uses CUDA sincos: the oracle gets the device's coordinates
         ro = np.arange(m + 1, dtype=np.int64) * (nv + 1)
         arr = og.OGArray(og.POLYGON, xy, geom_off=np.arange(m + 1, dtype=np.int64), ring_off=ro)
@@ -629,9 +706,7 @@ class HullWorkload:
         got_off = hro[: m + 1].cpu().numpy()
         assert np.array_equal(got_off, want_off), "hull ring offsets differ from the oracle"
         assert np.array_equal(hxy[: int(got_off[-1])].cpu().numpy(), want_xy), "hull rings differ from the oracle (vertex set or order)"
-        mv = torch.empty((self.nc, 2), dtype=torch.float64, device=e.dev)
-        E.check(e.ctx.lib.gpl_array_copy_out(e.ctx._h, self.moved._h, C.c_void_p(mv.data_ptr()), None, None, None, None, E.GPL_DEVICE))
-        e.stream.synchronize()
+        mv = self.moved_coords()
         assert np.array_equal(mv[: m * (nv + 1)].cpu().numpy(), og.affine_transform(xy, self.MATRIX, threads=len(all_cpus()))), "affine_transform is not bit-exact"
         self.write_bytes = self.nc * COORD_BYTES + hv.n_coords * COORD_BYTES
         return {"rows_checked_per_rank": m, "hull_rings_bit_identical": True, "affine_bit_exact": True, "hull_mean_vertices": hv.n_coords / max(1, self.g)}
@@ -767,7 +842,12 @@ def _main(out):
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-verify", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed to DIR/<name>.npy (see above)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the GPU path computed: it needs --impl b200")
     if args.workload in ("c3",):
         args.verify_rows = min(args.verify_rows, 2_000_000)
     if args.workload in ("c5",):
@@ -847,6 +927,9 @@ def _main(out):
         env.ctx.kernel_timing(False)
         # the dominant kernel alone when the library timed it (the join workloads), else the events around the op calls
         dom_ms = kt_ms / kt_n if kt_n else statistics.mean(k_ms)
+
+        if args.dump_outputs and env.rank == 0:
+            write_outputs(args.dump_outputs, wl.outputs())
 
         verify = None
         if not args.no_verify:

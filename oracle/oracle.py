@@ -34,9 +34,14 @@ class _OgArray(C.Structure):
 
 
 def _cpu_signature():
-    """identifies the host CPU (model + ISA flags): a -march=native build is only valid where it was made"""
+    """identifies the host CPU (model + ISA flags) and the oracle's source: a -march=native build is only valid where it
+    was made, and only for the source it was made from"""
     import hashlib
 
+    h = hashlib.sha1()
+    for name in ("geo_oracle.c", "geo_oracle.h", "Makefile"):
+        with open(os.path.join(_HERE, name), "rb") as f:
+            h.update(f.read())
     model, flags = "", ""
     try:
         with open("/proc/cpuinfo") as f:
@@ -49,7 +54,44 @@ def _cpu_signature():
                     break
     except OSError:
         pass
-    return model, hashlib.sha1((model + "|" + flags).encode()).hexdigest()[:12]
+    h.update((model + "|" + flags).encode())
+    return model, h.hexdigest()[:12]
+
+
+def _private_dir(path: str) -> str:
+    """create `path` if needed and return it, but only if it is a real directory (not a link) that belongs to this
+    user and that no one else can enter: the temporary directory is shared, and a library found there gets loaded"""
+    import stat
+
+    os.makedirs(path, mode=0o700, exist_ok=True)
+    st = os.lstat(path)
+    if not stat.S_ISDIR(st.st_mode) or st.st_uid != os.getuid() or st.st_mode & 0o077:
+        raise PermissionError(f"{path} is not a directory private to this user; the native oracle is not cached there")
+    return path
+
+
+def _build_native(sig: str) -> str:
+    """Compile the -march=native build for this host into a private per-user temporary directory (the source tree
+    may be read-only) and return its directory.  Each build goes to a fresh directory that is then renamed into
+    place, so that concurrent processes never load a half-written library."""
+    import shutil
+    import tempfile
+
+    base = _private_dir(os.path.join(tempfile.gettempdir(), f"geo_oracle-{os.getuid()}"))
+    ndir = os.path.join(base, sig)
+    if os.path.exists(os.path.join(ndir, "flags.txt")):
+        return ndir
+    tmp = tempfile.mkdtemp(dir=base)
+    try:
+        subprocess.check_call(["make", "-C", _HERE, "-s", "native", f"NATIVE_DIR={tmp}"],
+                              stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
+        os.rename(tmp, ndir)
+    except OSError:
+        if not os.path.exists(os.path.join(ndir, "flags.txt")):  # not another process's finished build
+            raise
+    finally:
+        shutil.rmtree(tmp, ignore_errors=True)
+    return ndir
 
 
 _build_info = {"flags": None, "cpu": None, "so": None, "native": False}
@@ -69,14 +111,10 @@ def build(force: bool = False) -> str:
     except Exception:
         _build_info["flags"] = "portable build (flags unknown)"
     if os.environ.get("GEO_ORACLE_NATIVE", "1") != "0":
-        ndir = os.path.join(_HERE, "_native", sig)
-        nso = os.path.join(ndir, "libgeo_oracle.so")
         try:
-            if force or not os.path.exists(nso) or os.path.getmtime(nso) < os.path.getmtime(src):
-                subprocess.check_call(["make", "-C", _HERE, "-s", "native", f"NATIVE_DIR={os.path.join('_native', sig)}"],
-                                      stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
+            ndir = _build_native(sig)
             with open(os.path.join(ndir, "flags.txt")) as f:
-                _build_info.update(flags=f.read().strip(), so=nso, native=True)
+                _build_info.update(flags=f.read().strip(), so=os.path.join(ndir, "libgeo_oracle.so"), native=True)
         except Exception:
             pass  # no compiler on this host: the portable build stands
     return _build_info["so"]

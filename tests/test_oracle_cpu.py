@@ -446,3 +446,32 @@ def test_area_centroid_length_envelope_against_exact_rational(og, conv):
 
             want_len = math.fsum(math.hypot(b[0] - a[0], b[1] - a[1]) for rings in parts for a, b in zip(rings[0][:-1], rings[0][1:]))
             assert abs(length[i] - want_len) <= 1e-12 * want_len
+
+
+def test_native_oracle_cache_is_private(tmp_path, monkeypatch):
+    """the -march=native oracle is cached under the shared temporary directory: a cache directory that is a link, or that
+    others can enter, is refused instead of loading a library planted there; a private one is built once and reused"""
+    import tempfile
+
+    from oracle import oracle
+
+    monkeypatch.setattr(tempfile, "tempdir", str(tmp_path))
+    base = tmp_path / f"geo_oracle-{os.getuid()}"
+    planted = tmp_path / "planted"
+    (planted / "sig").mkdir(parents=True)
+    (planted / "sig" / "flags.txt").write_text("planted")
+    planted.chmod(0o700)
+    base.symlink_to(planted)
+    with pytest.raises(PermissionError):
+        oracle._build_native("sig")
+    base.unlink()
+    planted.chmod(0o755)
+    planted.rename(base)
+    with pytest.raises(PermissionError):
+        oracle._build_native("sig")
+    base.chmod(0o700)
+    built = oracle._build_native("fresh")
+    assert built == str(base / "fresh") and (base / "fresh" / "libgeo_oracle.so").is_file()
+    assert "-march=native" in (base / "fresh" / "flags.txt").read_text()
+    assert sorted(p.name for p in base.iterdir()) == ["fresh", "sig"]  # no half-built directory left behind
+    assert oracle._build_native("fresh") == built
