@@ -14,7 +14,8 @@ import ctypes as C
 import os
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-# GEOPOLARS_B200_LIB: load another build of the same library (kernel-variant experiments)
+# GEOPOLARS_B200_LIB: load another build of the same library.  The library reads no environment itself, so this is how
+# two builds (say, before and after a kernel change) are compared on the same inputs.
 SO_PATH = os.environ.get("GEOPOLARS_B200_LIB") or os.path.join(_HERE, "libgeopolars_b200.so")
 
 GPL_HOST, GPL_DEVICE = 0, 1

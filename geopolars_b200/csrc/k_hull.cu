@@ -18,7 +18,6 @@
 // for element, so even exact ties for "farthest" resolve like the restated geo code (Iterator::max_by keeps the
 // LAST maximal element of the slice).  DESIGN.md "convex_hull".
 #include <math.h>
-#include <stdlib.h>
 
 #include "common.cuh"
 #include "scan.cuh"
@@ -294,7 +293,7 @@ __global__ void __launch_bounds__(kHullWarps * 32, SMEM ? 5 : 2) k_hull(int type
     tmp = P + cap;
     const int64_t n_warps = (int64_t)gridDim.x * kHullWarps;
     for (int64_t g = (int64_t)blockIdx.x * kHullWarps + wid; g < n_geoms; g += n_warps) {
-        if (only && !only[g]) continue;  // the level-wise kernel finished this geometry
+        if (!only[g]) continue;  // the level-wise kernel finished this geometry
         Emitter<WRITE> em;
         em.n = 0;
         em.out = WRITE ? out_xy + out_off[g] : nullptr;
@@ -720,16 +719,12 @@ extern "C" int gpl_convex_hull(gpl_ctx *ctx, const gpl_array *in, gpl_array **ou
     GPL_TRY(workspace.get(ctx, (stack_bytes + (use_smem ? 0 : stage_bytes)) * kHullWarps * (size_t)grid));
     const size_t dyn = use_smem ? smem_bytes : 0;
     // The level-wise kernel takes every geometry it can (4 <= coordinates <= fast_cap, finite, no arg-max tie between distinct
-    // points); what it flags in `redo` is recomputed by the order-exact kernel.  GPL_HULL_FAST=0 runs the exact kernel alone.
-    static const bool fast_enabled = [] {
-        const char *e = getenv("GPL_HULL_FAST");
-        return !e || atoi(e) != 0;
-    }();
+    // points); what it flags in `redo` is recomputed by the order-exact kernel.
     const int32_t fast_cap = (int32_t)((std::min<unsigned long long>(std::max<unsigned long long>(h_max, 4), 1024) + 1) & ~1ULL);
     const size_t fast_smem = HullFastLayout::bytes(fast_cap) * kHullWarps;
     int fast_grid = 1;
     Scratch<uint8_t> redo;
-    if (fast_enabled && n > 0) {
+    if (n > 0) {
         GPL_TRY(redo.get(ctx, (size_t)n));
         GPL_CUDA(cudaFuncSetAttribute(k_hull_fast<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fast_smem));
         GPL_CUDA(cudaFuncSetAttribute(k_hull_fast<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fast_smem));
@@ -741,23 +736,19 @@ extern "C" int gpl_convex_hull(gpl_ctx *ctx, const gpl_array *in, gpl_array **ou
     // pass: 0 = count only, 1 = write.  `off`/`dst` are the ring offsets and the output buffer of a writing pass.
     auto launch = [&](bool write, int64_t *cnt, const int64_t *off, double2 *dst) -> int {
         if (n == 0) return GPL_OK;
-        const uint8_t *only = nullptr;
-        if (fast_enabled) {
-            if (write)
-                k_hull_fast<true><<<fast_grid, kHullWarps * 32, fast_smem, ctx->stream>>>(in->type, n, xy, in->geom_off, in->part_off, in->ring_off, in->validity,
-                                                                                   fast_cap, cnt, off, dst, redo.p);
-            else
-                k_hull_fast<false><<<fast_grid, kHullWarps * 32, fast_smem, ctx->stream>>>(in->type, n, xy, in->geom_off, in->part_off, in->ring_off, in->validity,
-                                                                                    fast_cap, cnt, off, dst, redo.p);
-            ctx->launches++;
-            only = redo.p;
-        }
+        if (write)
+            k_hull_fast<true><<<fast_grid, kHullWarps * 32, fast_smem, ctx->stream>>>(in->type, n, xy, in->geom_off, in->part_off, in->ring_off, in->validity,
+                                                                               fast_cap, cnt, off, dst, redo.p);
+        else
+            k_hull_fast<false><<<fast_grid, kHullWarps * 32, fast_smem, ctx->stream>>>(in->type, n, xy, in->geom_off, in->part_off, in->ring_off, in->validity,
+                                                                                fast_cap, cnt, off, dst, redo.p);
+        ctx->launches++;
         if (use_smem) {
-            if (write) k_hull<true, true><<<grid, kHullWarps * 32, dyn, ctx->stream>>>(in->type, n, xy, in->geom_off, in->part_off, in->ring_off, in->validity, cap, workspace.p, cnt, off, dst, only);
-            else k_hull<false, true><<<grid, kHullWarps * 32, dyn, ctx->stream>>>(in->type, n, xy, in->geom_off, in->part_off, in->ring_off, in->validity, cap, workspace.p, cnt, off, dst, only);
+            if (write) k_hull<true, true><<<grid, kHullWarps * 32, dyn, ctx->stream>>>(in->type, n, xy, in->geom_off, in->part_off, in->ring_off, in->validity, cap, workspace.p, cnt, off, dst, redo.p);
+            else k_hull<false, true><<<grid, kHullWarps * 32, dyn, ctx->stream>>>(in->type, n, xy, in->geom_off, in->part_off, in->ring_off, in->validity, cap, workspace.p, cnt, off, dst, redo.p);
         } else {
-            if (write) k_hull<true, false><<<grid, kHullWarps * 32, 0, ctx->stream>>>(in->type, n, xy, in->geom_off, in->part_off, in->ring_off, in->validity, cap, workspace.p, cnt, off, dst, only);
-            else k_hull<false, false><<<grid, kHullWarps * 32, 0, ctx->stream>>>(in->type, n, xy, in->geom_off, in->part_off, in->ring_off, in->validity, cap, workspace.p, cnt, off, dst, only);
+            if (write) k_hull<true, false><<<grid, kHullWarps * 32, 0, ctx->stream>>>(in->type, n, xy, in->geom_off, in->part_off, in->ring_off, in->validity, cap, workspace.p, cnt, off, dst, redo.p);
+            else k_hull<false, false><<<grid, kHullWarps * 32, 0, ctx->stream>>>(in->type, n, xy, in->geom_off, in->part_off, in->ring_off, in->validity, cap, workspace.p, cnt, off, dst, redo.p);
         }
         ctx->launches++;
         GPL_CUDA(cudaGetLastError());

@@ -44,7 +44,6 @@
 // the cell.  Points on or near a boundary always take the walk, i.e. geo's own rule.
 #include <cooperative_groups.h>
 #include <math.h>
-#include <stdlib.h>
 #include <string.h>
 
 #include "common.cuh"
@@ -97,11 +96,8 @@ static_assert(sizeof(CellRec) == 32, "CellRec must be one sector");
 
 constexpr int32_t kFastBit = 1 << 30;  // PartLite::nb_flags: the CellRec points at the FP32 fast table
 constexpr int kFastCShift = 24;        // bits 24..29: C/2 (C = 16-byte records per bucket incl. header, even)
-#ifndef GPL_FAST_LIST
-#define GPL_FAST_LIST 6
-#endif
-constexpr int kFastListRecs = GPL_FAST_LIST;  // records per fast list: header + edges, even (see the FP32 fast table below)
-static_assert(GPL_FAST_LIST % 2 == 0 && GPL_FAST_LIST >= 2 && GPL_FAST_LIST <= 8, "fast list = 1..4 sectors");
+constexpr int kFastListRecs = 6;  // records per fast list: header + edges, even (see the FP32 fast table below)
+static_assert(kFastListRecs % 2 == 0 && kFastListRecs >= 2 && kFastListRecs <= 8, "fast list = 1..4 sectors");
 constexpr int kFastMaxCount = 120;  // longest bucket list a fast part may have
 
 struct __align__(32) EdgeRec {  // one L2 sector
@@ -189,6 +185,10 @@ __device__ __forceinline__ double ord_dec(unsigned long long u) {
 // ------------------------------------------------------------------------------------------------
 constexpr int kBuildThreads = 256;
 constexpr int kMaxBuildCtas = 1024;
+// edge slots per y-bucket x 100.  Round 1 (every point walks; kernel ms): 133: 2.18, 200: 2.03, 300: 1.95, 400: 1.98,
+// 500: 2.07.  Round 2 (12 % of the points walk): 300: query 0.837 / build 0.54 ms, 600: query 0.842 / build 0.42 ms —
+// half as many buckets to finish, the same query time.
+constexpr int kSlotsX100 = 600;
 
 enum {  // BuildArgs::acc slots (unsigned long long each, zeroed by the host before the count kernel)
     ACC_XMIN = 0, ACC_YMIN, ACC_XMAX, ACC_YMAX,  // union bbox, order-preserving encodings (min as max of the complement)
@@ -201,7 +201,6 @@ struct BuildArgs {
     const double2 *xy;
     const int64_t *geom_off, *part_off, *ring_off;
     const uint8_t *validity;
-    int slots_x100;
     int32_t G, rs;
     int64_t n_cells, NB_cap;
     // phase 1 (scratch)
@@ -414,9 +413,9 @@ __device__ void ph_headers(const BuildArgs &a, double *sm_box /* 4 x 8 */) {
         if (lane == 0) {
             PartHeader h;
             h.xmin = x0, h.ymin = y0, h.xmax = x1, h.ymax = y1;
-            // ~3 edge slots per y-bucket (slots_x100): on the config-2 stars a bucket lists ~9 of the 64 edges, and
+            // ~6 edge slots per y-bucket (kSlotsX100): on the config-2 stars a bucket lists ~9 of the 64 edges, and
             // each of its two one-sided lists (FP32 table) ~4.5.
-            int64_t nb = valid ? (n_slots * 100 + a.slots_x100 - 1) / a.slots_x100 : 0;
+            int64_t nb = valid ? (n_slots * 100 + kSlotsX100 - 1) / kSlotsX100 : 0;
             if (nb < 1) nb = valid ? 1 : 0;
             if (nb > 4096) nb = 4096;
             const float yminf = __double2float_rd(y0);
@@ -1202,15 +1201,8 @@ __device__ __forceinline__ int64_t coarse_cell(const GridParams &g, double px, d
 }
 
 // 256-bit loads (sm_100: LDG.E.256): one instruction, one L1 wavefront per distinct line
-#ifndef GPL_PIP_NOALLOC
-#define GPL_PIP_NOALLOC 0
-#endif
 __device__ __forceinline__ void ld256(const void *p, double &a, double &b, double &c, double &d) {
-#if GPL_PIP_NOALLOC
-    asm("ld.global.nc.L1::no_allocate.v4.f64 {%0,%1,%2,%3}, [%4];" : "=d"(a), "=d"(b), "=d"(c), "=d"(d) : "l"(p));
-#else
     asm("ld.global.nc.v4.f64 {%0,%1,%2,%3}, [%4];" : "=d"(a), "=d"(b), "=d"(c), "=d"(d) : "l"(p));
-#endif
 }
 __device__ __forceinline__ void ld256(const void *p, int32_t (&r)[8]) {
     asm("ld.global.nc.v8.b32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
@@ -1242,13 +1234,7 @@ __device__ __forceinline__ void edge_rule_fast(double sx, double sy, double ex, 
     wn += (int)(a && !b && det > 0.0) - (int)(!a && b && det < 0.0);
 }
 
-#ifndef GPL_PIP_MINB
-#define GPL_PIP_MINB 3
-#endif
-#ifndef GPL_PIP_THREADS
-#define GPL_PIP_THREADS 256
-#endif
-constexpr int kQueryThreads = GPL_PIP_THREADS;
+constexpr int kQueryThreads = 256;
 constexpr int32_t kDeferred = -2;  // first_id marker: "the fast filter could not decide, see k_pip_deferred"
 
 __device__ __forceinline__ void unpack_lite(const int32_t *r, PartLite &l) {
@@ -1391,10 +1377,11 @@ __device__ __forceinline__ bool fast_walk(const float4 *__restrict__ fast, const
 }
 
 // The walk of ONE point that lies inside the union bbox: coarse cell -> candidates -> edge lists.
-// MODE 0: first (lowest containing row or -1) and cnt; `undecided` = a filter could not certify something: the caller
-//         defers the point to the exact kernel.
-// MODE 1: write every (point, polygon) pair at lhs/rhs[w...]; undecided candidates are resolved in place with the
-//         exact predicate (this mode is not the throughput path).
+// MODE 0 (k_pip_stream): first (lowest containing row or -1) and cnt (all containing rows when want_count, else the walk
+//         stops at the first hit); `undecided` = a filter could not certify something: the caller defers the point to
+//         the exact kernel.
+// MODE 1 (k_pip_pairs): write every (point, polygon) pair at lhs/rhs[w...]; undecided candidates are resolved in place
+//         with the exact predicate (this mode is not the throughput path).
 // LEAN (MODE 0 only): every part of the index is a plain POLYGON with FP32 lists (the host checks it), so the
 // f64 bucket walk is compiled out and every candidate runs the FP32 walk.  A candidate that would still need the
 // f64 walk is deferred (cannot happen when the host check holds; kept so that the kernel is correct on any index).
@@ -1501,22 +1488,14 @@ __device__ __forceinline__ void walk_point(const IndexView &ix, const double2 p,
     }
 }
 
-#ifndef GPL_PIP_LEAN_MINB
-#define GPL_PIP_LEAN_MINB 4
-#endif
-// Round-1 kernel, kept for MODE 1 (pair lists) and as the A/B baseline (GPL_PIP_LEGACY=1): one thread per point,
-// every point walks.  32 consecutive points per warp (coalesced 512-byte read, software-prefetched one grid stride
-// ahead).
-template <int MODE, bool LEAN = false>
-__global__ void __launch_bounds__(kQueryThreads, LEAN ? GPL_PIP_LEAN_MINB : GPL_PIP_MINB) k_pip_query(const IndexView ix, const double2 *__restrict__ pts,
-                                                                           const uint8_t *__restrict__ pts_validity,
-                                                                           int64_t n_pts, int32_t *__restrict__ first_id,
-                                                                           int32_t *__restrict__ count,
-                                                                           const int64_t *__restrict__ pair_off,
-                                                                           uint64_t *__restrict__ lhs, uint64_t *__restrict__ rhs,
-                                                                           int64_t point_base,
-                                                                           unsigned long long *__restrict__ n_deferred,
-                                                                           uint32_t *__restrict__ deferred_list, uint32_t list_cap) {
+// Pair lists: the (point, polygon) pairs of point i go to lhs/rhs[pair_off[i]...] (the offsets are the exclusive scan of
+// the per-point counts of a k_pip_stream pass).  One thread per point, every point walks (round 1's query kernel, MODE 1
+// of walk_point).  32 consecutive points per warp (coalesced 512-byte read, software-prefetched one grid stride ahead).
+constexpr int kPairsMinBlocks = 3;
+__global__ void __launch_bounds__(kQueryThreads, kPairsMinBlocks) k_pip_pairs(const IndexView ix, const double2 *__restrict__ pts,
+                                                                               const uint8_t *__restrict__ pts_validity, int64_t n_pts,
+                                                                               const int64_t *__restrict__ pair_off,
+                                                                               uint64_t *__restrict__ lhs, uint64_t *__restrict__ rhs) {
     const GridParams &g = ix.grid;
     const int64_t stride = (int64_t)gridDim.x * kQueryThreads;
     int64_t i = (int64_t)blockIdx.x * kQueryThreads + threadIdx.x;
@@ -1529,18 +1508,7 @@ __global__ void __launch_bounds__(kQueryThreads, LEAN ? GPL_PIP_LEAN_MINB : GPL_
         if (ok && pts_validity) ok = bit_get(pts_validity, i);
         int32_t first = -1, cnt = 0;
         bool undecided = false;
-        if (ok)
-            walk_point<MODE, LEAN>(ix, p, count != nullptr, first, cnt, undecided, (uint64_t)(point_base + i), MODE == 1 ? pair_off[i] : 0, lhs,
-                                   rhs);
-        if (MODE == 0) {
-            if (undecided) {
-                first = kDeferred;
-                const unsigned long long slot = atomicAdd(n_deferred, 1ULL);
-                if (slot < list_cap) deferred_list[slot] = (uint32_t)i;  // chunk-relative index (chunks are < 2^32 points)
-            }
-            __stcs(first_id + i, first);
-            if (count) __stcs(count + i, cnt);
-        }
+        if (ok) walk_point<1, false>(ix, p, false, first, cnt, undecided, (uint64_t)i, pair_off[i], lhs, rhs);
     }
 }
 
@@ -1561,20 +1529,12 @@ struct __align__(16) StreamSmem {
     double2 q_pts[kStreamWarps][kQueueCap];
     uint32_t q_idx[kStreamWarps][kQueueCap];
 };
-#ifndef GPL_PIP_STREAM_MINB
-#define GPL_PIP_STREAM_MINB 3
-#endif
-__device__ __forceinline__ void ld256s(const double2 *p, double2 &a, double2 &b) {  // read-once stream: evict first
-    asm volatile("ld.global.cs.v4.f64 {%0,%1,%2,%3}, [%4];" : "=d"(a.x), "=d"(a.y), "=d"(b.x), "=d"(b.y) : "l"(p));
-}
-// cache-hint variants (GPL_PIP_LD_HINTS, A/B switch): the point stream without an L1 line (L2: evict first), the raster gather
-// (20 MB of random 8-byte words: no reuse an L1 could catch) without one — leaves the L1 to the cell / part / edge records.
-__device__ __forceinline__ void ld256s_na(const double2 *p, double2 &a, double2 &b, unsigned long long pol) {
-    asm volatile("ld.global.L1::no_allocate.L2::cache_hint.v4.f64 {%0,%1,%2,%3}, [%4], %5;"
-                 : "=d"(a.x), "=d"(a.y), "=d"(b.x), "=d"(b.y)
-                 : "l"(p), "l"(pol));
-}
-__device__ __forceinline__ void ld256s_na0(const double2 *p, double2 &a, double2 &b) {
+constexpr int kStreamMinBlocks = 3;
+// The point stream and the raster gather (20 MB of random 8-byte words: no reuse an L1 could catch) are loaded without an
+// L1 line, which leaves the L1 to the cell / part / edge records of the walk.  Query ms, config 2 / config 4: plain loads
+// 0.846 / 0.856; raster gather L1::no_allocate 0.821 / 0.832; both 0.819 / 0.827; both plus an L2 evict-first policy on the
+// stream 0.812 / 0.955.
+__device__ __forceinline__ void ld256s_na(const double2 *p, double2 &a, double2 &b) {
     asm volatile("ld.global.L1::no_allocate.v4.f64 {%0,%1,%2,%3}, [%4];" : "=d"(a.x), "=d"(a.y), "=d"(b.x), "=d"(b.y) : "l"(p));
 }
 __device__ __forceinline__ uint2 ldg_na(const uint2 *p) {
@@ -1582,34 +1542,15 @@ __device__ __forceinline__ uint2 ldg_na(const uint2 *p) {
     asm("ld.global.nc.L1::no_allocate.v2.u32 {%0,%1}, [%2];" : "=r"(v.x), "=r"(v.y) : "l"(p));
     return v;
 }
-// HIST: per-polygon hit counts (config 4's all-reduce input) in the same pass: 32-bit bins privatised per CTA in shared
-// memory behind the queues, flushed with one 64-bit global atomic per non-zero bin when the CTA retires.
-// CSM: the rows of candidate #0 of every coarse cell (raster code 1: 36 % of config 2's points) staged in shared memory —
-// the 8-byte gather from the L1-resident table cost L1/TEX tag wavefronts, the limiter of this kernel (ncu: l1tex 84 %).
-template <bool LEAN, bool HIST, bool CSM>
-__global__ void __launch_bounds__(kQueryThreads, GPL_PIP_STREAM_MINB) k_pip_stream(const IndexView ix, const double2 *__restrict__ pts,
-                                                                                  const uint8_t *__restrict__ pts_validity, int64_t n_pts,
-                                                                                  int32_t *__restrict__ first_id, int32_t *__restrict__ count,
-                                                                                  unsigned long long *__restrict__ n_deferred,
-                                                                                  uint32_t *__restrict__ deferred_list, uint32_t list_cap,
-                                                                                  int vec_ok, unsigned long long *__restrict__ hist, int32_t n_bins,
-                                                                                  int hints) {
+template <bool LEAN>
+__global__ void __launch_bounds__(kQueryThreads, kStreamMinBlocks) k_pip_stream(const IndexView ix, const double2 *__restrict__ pts,
+                                                                               const uint8_t *__restrict__ pts_validity, int64_t n_pts,
+                                                                               int32_t *__restrict__ first_id, int32_t *__restrict__ count,
+                                                                               unsigned long long *__restrict__ n_deferred,
+                                                                               uint32_t *__restrict__ deferred_list, uint32_t list_cap,
+                                                                               int vec_ok) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
-    unsigned long long pol_ef = 0ULL;
-    if (hints & 2) asm("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol_ef));
-    const bool raster_na = (hints & 1) != 0, pts_na = (hints & 2) != 0;
     StreamSmem &sm = *reinterpret_cast<StreamSmem *>(smem_raw);
-    unsigned int *bins = reinterpret_cast<unsigned int *>(smem_raw + sizeof(StreamSmem));
-    int32_t *cand0 = reinterpret_cast<int32_t *>(smem_raw + sizeof(StreamSmem));  // HIST and CSM are never combined
-    if (HIST) {
-        for (int32_t b = threadIdx.x; b < n_bins; b += kQueryThreads) bins[b] = 0u;
-        __syncthreads();
-    }
-    if (CSM) {
-        const int32_t n_cells = ix.grid.gx * ix.grid.gy;
-        for (int32_t c = threadIdx.x; c < n_cells; c += kQueryThreads) cand0[c] = __ldg(&ix.cand01[c].x);
-        __syncthreads();
-    }
     const GridParams &g = ix.grid;
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
     double2 *q_pts = sm.q_pts[wid];
@@ -1636,7 +1577,6 @@ __global__ void __launch_bounds__(kQueryThreads, GPL_PIP_STREAM_MINB) k_pip_stre
             }
             first_id[idx] = first;
             if (want_count) count[idx] = cnt;
-            if (HIST && first >= 0 && first < n_bins) atomicAdd(&bins[first], 1u);
         }
     };
 
@@ -1646,16 +1586,8 @@ __global__ void __launch_bounds__(kQueryThreads, GPL_PIP_STREAM_MINB) k_pip_stre
     auto load_tile = [&](int64_t t, double2 (&dst)[4]) {
         const int64_t base = t * kTilePts;
         if (vec_ok && base + kTilePts <= n_pts) {
-            if (pts_na) {
-                ld256s_na(pts + base + 2 * lane, dst[0], dst[1], pol_ef);
-                ld256s_na(pts + base + 64 + 2 * lane, dst[2], dst[3], pol_ef);
-            } else if (hints & 4) {
-                ld256s_na0(pts + base + 2 * lane, dst[0], dst[1]);
-                ld256s_na0(pts + base + 64 + 2 * lane, dst[2], dst[3]);
-            } else {
-                ld256s(pts + base + 2 * lane, dst[0], dst[1]);
-                ld256s(pts + base + 64 + 2 * lane, dst[2], dst[3]);
-            }
+            ld256s_na(pts + base + 2 * lane, dst[0], dst[1]);
+            ld256s_na(pts + base + 64 + 2 * lane, dst[2], dst[3]);
         } else {
 #pragma unroll
             for (int k = 0; k < 4; ++k) {
@@ -1683,7 +1615,7 @@ __global__ void __launch_bounds__(kQueryThreads, GPL_PIP_STREAM_MINB) k_pip_stre
             if (ok[k] && pts_validity) ok[k] = bit_get(pts_validity, i);
             fx[k] = fine_index(p[k].x, g.x0, g.inv_fw, g.fgx), fy[k] = fine_index(p[k].y, g.y0, g.inv_fh, g.fgy);
             const uint2 *wp = ix.raster + (int64_t)fy[k] * g.wpr + (fx[k] >> 4);
-            word[k] = ok[k] ? (raster_na ? ldg_na(wp) : __ldg(wp)) : make_uint2(0u, 0u);
+            word[k] = ok[k] ? ldg_na(wp) : make_uint2(0u, 0u);
         }
         // stage 2: codes -> ids
         int32_t id[4];
@@ -1696,13 +1628,11 @@ __global__ void __launch_bounds__(kQueryThreads, GPL_PIP_STREAM_MINB) k_pip_stre
                 const int64_t cc = (int64_t)(fy[k] >> g.rs) * g.gx + (fx[k] >> g.rs);
                 if (code[k] == 1u && word[k].y != 0xfffffffeu) {
                     id[k] = (int32_t)word[k].y;  // the candidate's row travels with the codes: no second gather
-                } else if (CSM && code[k] == 1u) {
-                    id[k] = cand0[cc];
                 } else {
+                    // (staging the whole table in shared memory measured slower on config 2: 0.98 vs 0.90 ms)
                     const int2 cand = __ldg(ix.cand01 + cc);
                     id[k] = code[k] == 1u ? cand.x : cand.y;
                 }
-                if (HIST && id[k] >= 0 && id[k] < n_bins) atomicAdd(&bins[id[k]], 1u);
             }
         }
         // stage 3: ids out (the queued ones are overwritten by the walk)
@@ -1742,13 +1672,6 @@ __global__ void __launch_bounds__(kQueryThreads, GPL_PIP_STREAM_MINB) k_pip_stre
         }
     }
     if (qn > 0) walk_queued(lane, lane < qn);
-    if (HIST) {
-        __syncthreads();
-        for (int32_t b = threadIdx.x; b < n_bins; b += kQueryThreads) {
-            const unsigned int v = bins[b];
-            if (v) atomicAdd(hist + b, (unsigned long long)v);
-        }
-    }
 }
 
 // Exact re-evaluation of the points the walk marked kDeferred (those whose filters could not
@@ -1757,8 +1680,7 @@ __global__ void __launch_bounds__(kQueryThreads, GPL_PIP_STREAM_MINB) k_pip_stre
 // counter is zero.  One thread per deferred point, taken from the list the query kernel appended to; if
 // the list overflowed, the id column is scanned for the marker instead.
 __device__ __forceinline__ void deferred_point(const IndexView &ix, const double2 *__restrict__ pts, int64_t i,
-                                               int32_t *__restrict__ first_id, int32_t *__restrict__ count,
-                                               unsigned long long *__restrict__ hist) {
+                                               int32_t *__restrict__ first_id, int32_t *__restrict__ count) {
     const double2 p = pts[i];
     const CellRec cell = ix.cells[coarse_cell(ix.grid, p.x, p.y)];
     int32_t first = -1, cnt = 0, last_geom = -1;
@@ -1776,23 +1698,21 @@ __device__ __forceinline__ void deferred_point(const IndexView &ix, const double
     }
     first_id[i] = first;
     if (count) count[i] = cnt;
-    if (hist && first >= 0) atomicAdd(hist + first, 1ULL);  // the streaming kernel counted decided points only
 }
 __global__ void __launch_bounds__(256) k_pip_deferred(const IndexView ix, const double2 *__restrict__ pts, int64_t n_pts,
                                                       int32_t *__restrict__ first_id, int32_t *__restrict__ count,
                                                       unsigned long long *__restrict__ n_deferred,
                                                       const uint32_t *__restrict__ deferred_list, uint32_t list_cap,
-                                                      unsigned long long *__restrict__ n_deferred_total,
-                                                      unsigned long long *__restrict__ hist) {
+                                                      unsigned long long *__restrict__ n_deferred_total) {
     const unsigned long long nd = *n_deferred;
     if (nd == 0ULL) return;
     const int64_t stride = (int64_t)gridDim.x * blockDim.x;
     if (nd <= list_cap) {
         for (int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; k < (int64_t)nd; k += stride)
-            deferred_point(ix, pts, (int64_t)deferred_list[k], first_id, count, hist);
+            deferred_point(ix, pts, (int64_t)deferred_list[k], first_id, count);
     } else {
         for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n_pts; i += stride)
-            if (first_id[i] == kDeferred) deferred_point(ix, pts, i, first_id, count, hist);
+            if (first_id[i] == kDeferred) deferred_point(ix, pts, i, first_id, count);
     }
     if (blockIdx.x == 0 && threadIdx.x == 0 && n_deferred_total) atomicAdd(n_deferred_total, nd);
 }
@@ -1842,66 +1762,43 @@ static IndexView view_of(const gpl_pip_index *idx) {
     return v;
 }
 
-static int env_int(const char *name, int dflt) {
-    const char *e = getenv(name);
-    return e ? atoi(e) : dflt;
-}
-
-static int query_grid(int64_t n, bool lean = false) {
-    // persistent-style: 148 SMs x resident CTAs, grid-stride over the point stream
-    static const int per_sm_full = env_int("GPL_PIP_CTAS_PER_SM", 8);
-    static const int per_sm_lean = env_int("GPL_PIP_LEAN_CTAS_PER_SM", 2 * GPL_PIP_LEAN_MINB);  // two waves of the resident CTAs
-    const int per_sm = lean ? per_sm_lean : per_sm_full;
-    int64_t want = ceil_div(n, kQueryThreads);
-    return (int)std::max<int64_t>(1, std::min<int64_t>(want, (int64_t)kSMs * per_sm));
+// pair kernel: 148 SMs x 8 CTAs, grid-stride over the points
+static int pairs_grid(int64_t n) {
+    return (int)std::max<int64_t>(1, std::min<int64_t>(ceil_div(n, kQueryThreads), (int64_t)kSMs * 8));
 }
 // streaming kernel: exactly the resident CTAs (persistent warps, one tile of 128 points per warp and iteration)
-constexpr int32_t kHistFuseMaxBins = 12288;  // 48 KB of bins per CTA: three CTAs per SM still fit next to the queues
-template <bool LEAN, bool HIST, bool CSM>
-static int stream_grid(int64_t n, size_t smem_bytes) {
-    static size_t attr_bytes = 0;
-    if (smem_bytes > attr_bytes) {
-        cudaFuncSetAttribute(k_pip_stream<LEAN, HIST, CSM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes);
-        attr_bytes = smem_bytes;
-    }
-    int occ = 0;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_pip_stream<LEAN, HIST, CSM>, kQueryThreads, smem_bytes) != cudaSuccess || occ < 1) occ = 1;
-    (void)cudaGetLastError();
-    static const int cap = env_int("GPL_PIP_STREAM_CTAS_PER_SM", 0);
-    const int per_sm = cap > 0 ? std::min(cap, occ) : occ;
-    const int64_t want = ceil_div(ceil_div(n, kTilePts), kStreamWarps);
-    return (int)std::max<int64_t>(1, std::min<int64_t>(want, (int64_t)kSMs * per_sm));
-}
-constexpr int32_t kCandSmemMaxCells = 12288;  // 48 KB of candidate rows per CTA
-template <bool LEAN, bool HIST>
+template <bool LEAN>
 static void launch_stream(const IndexView &v, const double2 *pts, const uint8_t *val, int64_t m, int32_t *first, int32_t *cnt,
-                          const gpl_pip_index *idx, int vec_ok, unsigned long long *hist, int32_t n_bins, cudaStream_t stream) {
-    static const bool csm_enabled = env_int("GPL_PIP_CAND_SMEM", 0) != 0;  // measured slower on config 2 (0.98 vs 0.90 ms): opt-in
-    // bit 0: raster gather without an L1 line; bit 2: the point stream too; bit 1: the point stream too, plus an L2 evict-first
-    // policy.  Query ms, config 2 / config 4:  0: 0.846 / 0.856   1: 0.821 / 0.832   5: 0.819 / 0.827   3: 0.812 / 0.955
-    static const int hints = env_int("GPL_PIP_LD_HINTS", 5);
-    const int64_t n_cells = (int64_t)v.grid.gx * v.grid.gy;
-    if (!HIST && csm_enabled && n_cells <= kCandSmemMaxCells) {
-        const size_t smem = sizeof(StreamSmem) + sizeof(int32_t) * (size_t)n_cells;
-        k_pip_stream<LEAN, false, true><<<stream_grid<LEAN, false, true>(m, smem), kQueryThreads, smem, stream>>>(
-            v, pts, val, m, first, cnt, idx->n_deferred, idx->deferred_list, idx->deferred_cap, vec_ok, nullptr, 0, hints);
-        return;
-    }
-    const size_t smem = sizeof(StreamSmem) + (HIST ? sizeof(unsigned int) * (size_t)n_bins : 0);
-    k_pip_stream<LEAN, HIST, false><<<stream_grid<LEAN, HIST, false>(m, smem), kQueryThreads, smem, stream>>>(
-        v, pts, val, m, first, cnt, idx->n_deferred, idx->deferred_list, idx->deferred_cap, vec_ok, hist, n_bins, hints);
+                          const gpl_pip_index *idx, int vec_ok, cudaStream_t stream) {
+    constexpr size_t smem = sizeof(StreamSmem);
+    int occ = 0;
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_pip_stream<LEAN>, kQueryThreads, smem) != cudaSuccess || occ < 1) occ = 1;
+    (void)cudaGetLastError();
+    const int64_t want = ceil_div(ceil_div(m, kTilePts), kStreamWarps);
+    const int grid = (int)std::max<int64_t>(1, std::min<int64_t>(want, (int64_t)kSMs * occ));
+    k_pip_stream<LEAN><<<grid, kQueryThreads, smem, stream>>>(v, pts, val, m, first, cnt, idx->n_deferred, idx->deferred_list,
+                                                              idx->deferred_cap, vec_ok);
 }
-// hist (optional, device, n_geoms u64): += number of points whose first containing row is that polygon
+// counts[id] += 1 for every id in [0, n_polys) of the column ids[0, n)
+static int launch_histogram(gpl_ctx *ctx, const int32_t *ids, int64_t n, unsigned long long *counts, int64_t n_polys,
+                            cudaStream_t stream) {
+    const bool use_smem = n_polys <= kHistSmemBins;
+    const size_t dyn = use_smem ? sizeof(unsigned int) * (size_t)n_polys : 0;
+    if (dyn > 48 * 1024) GPL_CUDA(cudaFuncSetAttribute(k_histogram, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn));
+    const int per_sm = use_smem ? (int)std::max<size_t>(1, std::min<size_t>(4, (200 * 1024) / std::max<size_t>(dyn, 1))) : 4;
+    const int grid = (int)std::max<int64_t>(1, std::min<int64_t>(ceil_div(n, 2048), (int64_t)kSMs * per_sm));
+    k_histogram<<<grid, 512, dyn, stream>>>(ids, n, counts, n_polys, use_smem ? 1 : 0);
+    ctx->launches++;
+    return GPL_OK;
+}
+// hist (optional, device, n_geoms u64): += number of points whose first containing row is that polygon.  The counts are a
+// separate pass over the id column (k_histogram: 0.1 ms per 100 M ids): shared-memory bins fused into the streaming kernel
+// measured slower on config 2 (+0.22 ms).
 int pip_query(gpl_ctx *ctx, const gpl_pip_index *idx, const double *pts_dev, const uint8_t *validity_dev, int64_t n,
               int32_t *first_dev, int32_t *count_dev, cudaStream_t stream, unsigned long long *hist = nullptr) {
     if (n == 0) return GPL_OK;
-    // Per-polygon counts: a separate pass over the id column (k_histogram: 0.1 ms per 100 M ids) by default; the variant
-    // fused into the streaming kernel (shared-memory bins) measured slower on config 2 (+0.22 ms) and is opt-in.
-    static const bool fuse_enabled = env_int("GPL_PIP_FUSE_HIST", 0) != 0;
-    const bool fuse_hist = fuse_enabled && hist != nullptr && idx->n_geoms <= kHistFuseMaxBins;
     const double2 *pts = reinterpret_cast<const double2 *>(pts_dev);
     const IndexView v = view_of(idx);
-    static const bool legacy = env_int("GPL_PIP_LEGACY", 0) != 0;  // round-1 kernel: every point walks (A/B measurements)
     // the deferred list holds chunk-relative uint32 indices: process at most 2^31 points per launch pair
     const int64_t kMaxChunk = 1LL << 31;
     for (int64_t lo = 0; lo < n; lo += kMaxChunk) {
@@ -1918,46 +1815,20 @@ int pip_query(gpl_ctx *ctx, const gpl_pip_index *idx, const double *pts_dev, con
         GPL_CUDA(cudaMemsetAsync(idx->n_deferred, 0, sizeof(unsigned long long), stream));
         const uint8_t *val = validity_dev ? validity_dev + lo / 8 : nullptr;
         int32_t *cnt = count_dev ? count_dev + lo : nullptr;
-        if (legacy) {
-            if (idx->lean_ok)
-                k_pip_query<0, true><<<query_grid(m, true), kQueryThreads, 0, stream>>>(v, pts + lo, val, m, first_dev + lo, cnt, nullptr, nullptr,
-                                                                                    nullptr, lo, idx->n_deferred, idx->deferred_list,
-                                                                                    idx->deferred_cap);
-            else
-                k_pip_query<0, false><<<query_grid(m), kQueryThreads, 0, stream>>>(v, pts + lo, val, m, first_dev + lo, cnt, nullptr, nullptr,
-                                                                                     nullptr, lo, idx->n_deferred, idx->deferred_list,
-                                                                                     idx->deferred_cap);
-        } else {
-            cudaEvent_t t0 = nullptr, t1 = nullptr;
-            if (ctx->kt_on && ctx->kernel_timing_pair(&t0, &t1)) GPL_CUDA(cudaEventRecord(t0, stream));
-            // 256-bit point loads and 64-bit id stores need 32- / 8-byte aligned columns (cudaMalloc'd ones are)
-            const int vec_ok = ((reinterpret_cast<uintptr_t>(pts + lo) & 31) == 0 && (reinterpret_cast<uintptr_t>(first_dev + lo) & 7) == 0 &&
-                                (cnt == nullptr || (reinterpret_cast<uintptr_t>(cnt) & 7) == 0))
-                                   ? 1
-                                   : 0;
-            const int32_t nb = (int32_t)idx->n_geoms;
-            if (idx->lean_ok) {
-                if (fuse_hist) launch_stream<true, true>(v, pts + lo, val, m, first_dev + lo, cnt, idx, vec_ok, hist, nb, stream);
-                else launch_stream<true, false>(v, pts + lo, val, m, first_dev + lo, cnt, idx, vec_ok, nullptr, 0, stream);
-            } else {
-                if (fuse_hist) launch_stream<false, true>(v, pts + lo, val, m, first_dev + lo, cnt, idx, vec_ok, hist, nb, stream);
-                else launch_stream<false, false>(v, pts + lo, val, m, first_dev + lo, cnt, idx, vec_ok, nullptr, 0, stream);
-            }
-            if (t1) GPL_CUDA(cudaEventRecord(t1, stream));
-        }
-        const bool fused_here = fuse_hist && !legacy;
+        cudaEvent_t t0 = nullptr, t1 = nullptr;
+        if (ctx->kt_on && ctx->kernel_timing_pair(&t0, &t1)) GPL_CUDA(cudaEventRecord(t0, stream));
+        // 256-bit point loads and 64-bit id stores need 32- / 8-byte aligned columns (cudaMalloc'd ones are)
+        const int vec_ok = ((reinterpret_cast<uintptr_t>(pts + lo) & 31) == 0 && (reinterpret_cast<uintptr_t>(first_dev + lo) & 7) == 0 &&
+                            (cnt == nullptr || (reinterpret_cast<uintptr_t>(cnt) & 7) == 0))
+                               ? 1
+                               : 0;
+        if (idx->lean_ok) launch_stream<true>(v, pts + lo, val, m, first_dev + lo, cnt, idx, vec_ok, stream);
+        else launch_stream<false>(v, pts + lo, val, m, first_dev + lo, cnt, idx, vec_ok, stream);
+        if (t1) GPL_CUDA(cudaEventRecord(t1, stream));
         k_pip_deferred<<<kSMs * 8, 256, 0, stream>>>(v, pts + lo, m, first_dev + lo, cnt, idx->n_deferred, idx->deferred_list, idx->deferred_cap,
-                                                     idx->n_deferred + 1, fused_here ? hist : nullptr);
+                                                     idx->n_deferred + 1);
         ctx->launches += 2;
-        if (hist && !fused_here) {  // many polygons (or the legacy kernel): count from the id column
-            const bool use_smem = idx->n_geoms <= kHistSmemBins;
-            const size_t dyn = use_smem ? sizeof(unsigned int) * (size_t)idx->n_geoms : 0;
-            if (dyn > 48 * 1024) GPL_CUDA(cudaFuncSetAttribute(k_histogram, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn));
-            const int per_sm = use_smem ? (int)std::max<size_t>(1, std::min<size_t>(4, (200 * 1024) / std::max<size_t>(dyn, 1))) : 4;
-            const int grid = (int)std::max<int64_t>(1, std::min<int64_t>(ceil_div(m, 2048), (int64_t)kSMs * per_sm));
-            k_histogram<<<grid, 512, dyn, stream>>>(first_dev + lo, m, hist, idx->n_geoms, use_smem ? 1 : 0);
-            ctx->launches++;
-        }
+        if (hist) GPL_TRY(launch_histogram(ctx, first_dev + lo, m, hist, idx->n_geoms, stream));
     }
     GPL_CUDA(cudaGetLastError());
     return GPL_OK;
@@ -1968,14 +1839,13 @@ int pip_query(gpl_ctx *ctx, const gpl_pip_index *idx, const double *pts_dev, con
 using namespace gpl;
 
 // Keep the hot part of the index slab resident in the 126 MB L2 while 1.6 GB of points stream past it: mark it
-// as a persisting access-policy window on the context stream (the point loads are ld.global.cs,
-// i.e. evict-first).  Best effort: failures only cost performance.  The device-wide carve-out only ever grows while
-// the context lives and is restored by gpl_ctx_destroy; the window is dropped and the persisting lines are released
-// when the index that set them is freed (neither call waits for running kernels: they are cache hints).
+// as a persisting access-policy window on the context stream.  Best effort: failures only cost performance.  The
+// device-wide carve-out only ever grows while the context lives and is restored by gpl_ctx_destroy; the window is
+// dropped and the persisting lines are released when the index that set them is freed (neither call waits for running
+// kernels: they are cache hints).
 static void l2_pin(gpl_pip_index *idx, bool on) {
     gpl_ctx *ctx = idx->ctx;
-    static const bool enabled = env_int("GPL_L2_PIN", 1) != 0;
-    if (!enabled || ctx->l2_persist_max == 0 || ctx->l2_window_max == 0) return;
+    if (ctx->l2_persist_max == 0 || ctx->l2_window_max == 0) return;
     cudaStreamAttrValue attr;
     memset(&attr, 0, sizeof(attr));
     if (on) {
@@ -2124,24 +1994,17 @@ extern "C" int gpl_pip_index_build(gpl_ctx *ctx, const gpl_array *polys, gpl_pip
     cudaStream_t st = ctx->stream;
     static const int grid_count = coop_grid(k_pip_build_count), grid_fill = coop_grid(k_pip_build_fill);
 
-    // edge slots per y-bucket x 100.  Round 1 (every point walks; kernel ms): 133: 2.18, 200: 2.03, 300: 1.95, 400: 1.98,
-    // 500: 2.07.  Round 2 (12 % of the points walk): 300: query 0.837 / build 0.54 ms, 600: query 0.842 / build 0.42 ms —
-    // half as many buckets to finish, the same query time.
-    static const int slots_x100 = [] {
-        const int v = env_int("GPL_PIP_SLOTS_X100", 600);
-        return v >= 25 && v <= 6400 ? v : 600;
-    }();
     // coarse grid: about one cell per part.  Fine grid: 2^rs x 2^rs cells per coarse cell, as fine as a budget of
     // raster cells allows (8 bytes per 16 cells: 64 M cells = 32 MB, L2-resident next to the FP32 table), at most 2^7, and at
     // most 2^20 fine cells per axis (the error analysis of the raster assumes it).
+    constexpr int kRasterLog2Max = 7;
+    constexpr int64_t kRasterCells = 64LL << 20;
     int64_t G = (int64_t)ceil(sqrt((double)Pa));
     if (G < 1) G = 1;
     if (G > 2048) G = 2048;
     const int64_t n_cells = G * G;
-    static const int rs_max = std::min(7, std::max(0, env_int("GPL_PIP_RASTER_LOG2", 7)));
-    static const int64_t raster_budget = (int64_t)std::max(1, env_int("GPL_PIP_RASTER_MCELLS", 64)) << 20;
-    int rs = rs_max;
-    while (rs > 0 && (((G << rs) > (1 << 20)) || ((G << rs) * (G << rs) > raster_budget))) --rs;
+    int rs = kRasterLog2Max;
+    while (rs > 0 && (((G << rs) > (1 << 20)) || ((G << rs) * (G << rs) > kRasterCells))) --rs;
 
     // ---- phase 1 (scratch): bboxes, grid, cell counts, bucket counts, FP32 plan --------------------------------
     BuildArgs a;
@@ -2149,9 +2012,9 @@ extern "C" int gpl_pip_index_build(gpl_ctx *ctx, const gpl_array *polys, gpl_pip
     a.type = type, a.P = P, a.n_geoms = polys->n_geoms;
     a.xy = reinterpret_cast<const double2 *>(polys->xy);
     a.geom_off = polys->geom_off, a.part_off = polys->part_off, a.ring_off = polys->ring_off, a.validity = polys->validity;
-    a.slots_x100 = slots_x100, a.G = (int32_t)G, a.rs = rs, a.n_cells = n_cells;
-    // sum of n_buckets <= P + n_coords * 100 / slots_x100 + 1 without a host round trip
-    a.NB_cap = Pa + (polys->n_coords * 100) / slots_x100 + 1;
+    a.G = (int32_t)G, a.rs = rs, a.n_cells = n_cells;
+    // sum of n_buckets <= P + n_coords * 100 / kSlotsX100 + 1 without a host round trip
+    a.NB_cap = Pa + (polys->n_coords * 100) / kSlotsX100 + 1;
     Scratch<PartHeader> hdr;
     Scratch<GridParams> gp;
     Scratch<int32_t> nb, cell_count, cell_cursor, bcount, bcursor, fast_c, fast_slots;
@@ -2218,11 +2081,8 @@ extern "C" int gpl_pip_index_build(gpl_ctx *ctx, const gpl_array *polys, gpl_pip
     const size_t o_defer = carve(2 * sizeof(unsigned long long));
     const size_t o_phase = carve(16 * sizeof(unsigned long long));
     const bool all_fast = idx->n_fast > 0 && !idx->multi && !idx->any_holes;
-    {
-        static const bool lean_enabled = env_int("GPL_PIP_LEAN", 1) != 0;  // GPL_PIP_LEAN=0 forces the full walk (A/B measurements)
-        // POLYGON rows without holes, every valid part has FP32 lists (cells may hold several candidates)
-        idx->lean_ok = lean_enabled && all_fast && idx->n_not_fast == 0;
-    }
+    // POLYGON rows without holes, every valid part has FP32 lists (cells may hold several candidates)
+    idx->lean_ok = all_fast && idx->n_not_fast == 0;
     const size_t hot_mark = off;
     const size_t o_entries = carve(sizeof(EdgeRec) * (idx->n_entries + 1));
     const size_t o_ring = idx->any_holes ? carve(sizeof(int32_t) * (idx->n_entries + 1)) : 0;
@@ -2332,6 +2192,33 @@ extern "C" int gpl_contains_join_array(gpl_ctx *ctx, const gpl_pip_index *idx, c
     return GPL_OK;
 }
 
+// The (point, polygon) pair list of the device points pts[0, n) (validity optional; n > 0): the join with per-point
+// counts, their exclusive scan into pair offsets, the total read back (synchronises the stream), then
+// outputs(total, &lhs, &rhs) provides two device arrays of `total` elements, or leaves them NULL when no pairs are to be
+// written, and k_pip_pairs fills them.
+template <typename Outputs>
+static int contains_pairs(gpl_ctx *ctx, const gpl_pip_index *idx, const double *pts, const uint8_t *validity, int64_t n,
+                          Outputs outputs) {
+    Scratch<int32_t> ids, cnt;
+    Scratch<int64_t> off;
+    GPL_TRY(ids.get(ctx, (size_t)n));
+    GPL_TRY(cnt.get(ctx, (size_t)n));
+    GPL_TRY(off.get(ctx, (size_t)n + 2));
+    GPL_TRY(pip_query(ctx, idx, pts, validity, n, ids.p, cnt.p, ctx->stream));
+    GPL_TRY((exclusive_scan<int32_t, int64_t>(ctx, cnt.p, n, off.p, off.p + n + 1)));
+    int64_t total = 0;
+    GPL_CUDA(cudaMemcpyAsync(&total, off.p + n + 1, sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
+    GPL_CUDA(cudaStreamSynchronize(ctx->stream));
+    uint64_t *lhs = nullptr, *rhs = nullptr;
+    GPL_TRY(outputs(total, &lhs, &rhs));
+    if (lhs == nullptr) return GPL_OK;
+    k_pip_pairs<<<pairs_grid(n), kQueryThreads, 0, ctx->stream>>>(view_of(idx), reinterpret_cast<const double2 *>(pts), validity, n,
+                                                                  off.p, lhs, rhs);
+    ctx->launches++;
+    GPL_CUDA(cudaGetLastError());
+    return GPL_OK;
+}
+
 extern "C" int gpl_contains_join_pairs(gpl_ctx *ctx, const gpl_pip_index *idx, const double *points_xy, int64_t n_points,
                                        uint64_t *lhs, uint64_t *rhs, int64_t *n_pairs, int mem) {
     GPL_REQUIRE(ctx && idx && n_pairs, GPL_ERR_INVALID_ARG, "gpl_contains_join_pairs: NULL argument");
@@ -2347,38 +2234,25 @@ extern "C" int gpl_contains_join_pairs(gpl_ctx *ctx, const gpl_pip_index *idx, c
         GPL_CUDA(cudaMemcpyAsync(pts.p, points_xy, sizeof(double) * 2 * n_points, cudaMemcpyHostToDevice, ctx->stream));
         pdev = pts.p;
     }
-    Scratch<int32_t> ids, cnt;
-    Scratch<int64_t> off;
-    GPL_TRY(ids.get(ctx, (size_t)n_points));
-    GPL_TRY(cnt.get(ctx, (size_t)n_points));
-    GPL_TRY(off.get(ctx, (size_t)n_points + 2));
-    GPL_TRY(pip_query(ctx, idx, pdev, nullptr, n_points, ids.p, cnt.p, ctx->stream));
-    GPL_TRY((exclusive_scan<int32_t, int64_t>(ctx, cnt.p, n_points, off.p, off.p + n_points + 1)));
-    int64_t total = 0;
-    GPL_CUDA(cudaMemcpyAsync(&total, off.p + n_points + 1, sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
-    GPL_CUDA(cudaStreamSynchronize(ctx->stream));
-    if (lhs == nullptr || rhs == nullptr) {
-        *n_pairs = total;
-        return GPL_OK;
-    }
-    GPL_REQUIRE(*n_pairs >= total, GPL_ERR_INVALID_ARG, "pair buffers too small: need %lld, have %lld", (long long)total,
-                (long long)*n_pairs);
-    *n_pairs = total;
-    if (total == 0) return GPL_OK;
+    const bool count_only = lhs == nullptr || rhs == nullptr;
     Scratch<uint64_t> dl, dr;
-    uint64_t *pl = lhs, *pr = rhs;
-    if (mem == GPL_HOST) {
-        GPL_TRY(dl.get(ctx, (size_t)total));
-        GPL_TRY(dr.get(ctx, (size_t)total));
-        pl = dl.p, pr = dr.p;
-    }
-    k_pip_query<1><<<query_grid(n_points), kQueryThreads, 0, ctx->stream>>>(view_of(idx), reinterpret_cast<const double2 *>(pdev), nullptr,
-                                                                      n_points, nullptr, nullptr, off.p, pl, pr, 0, nullptr, nullptr, 0);
-    ctx->launches++;
-    GPL_CUDA(cudaGetLastError());
-    if (mem == GPL_HOST) {
-        GPL_CUDA(cudaMemcpyAsync(lhs, pl, sizeof(uint64_t) * total, cudaMemcpyDeviceToHost, ctx->stream));
-        GPL_CUDA(cudaMemcpyAsync(rhs, pr, sizeof(uint64_t) * total, cudaMemcpyDeviceToHost, ctx->stream));
+    GPL_TRY(contains_pairs(ctx, idx, pdev, nullptr, n_points, [&](int64_t total, uint64_t **pl, uint64_t **pr) -> int {
+        if (!count_only)
+            GPL_REQUIRE(*n_pairs >= total, GPL_ERR_INVALID_ARG, "pair buffers too small: need %lld, have %lld", (long long)total,
+                        (long long)*n_pairs);
+        *n_pairs = total;
+        if (count_only || total == 0) return GPL_OK;
+        *pl = lhs, *pr = rhs;
+        if (mem == GPL_HOST) {
+            GPL_TRY(dl.get(ctx, (size_t)total));
+            GPL_TRY(dr.get(ctx, (size_t)total));
+            *pl = dl.p, *pr = dr.p;
+        }
+        return GPL_OK;
+    }));
+    if (dl.p) {
+        GPL_CUDA(cudaMemcpyAsync(lhs, dl.p, sizeof(uint64_t) * *n_pairs, cudaMemcpyDeviceToHost, ctx->stream));
+        GPL_CUDA(cudaMemcpyAsync(rhs, dr.p, sizeof(uint64_t) * *n_pairs, cudaMemcpyDeviceToHost, ctx->stream));
     }
     GPL_CUDA(cudaStreamSynchronize(ctx->stream));
     return GPL_OK;
@@ -2399,27 +2273,17 @@ extern "C" int gpl_contains_join_pairs_array(gpl_ctx *ctx, const gpl_pip_index *
     *out = res;
     const int64_t n = points->n_geoms;
     if (n == 0) return GPL_OK;
-    Scratch<int32_t> ids, cnt;
-    Scratch<int64_t> off;
-    GPL_TRY(ids.get(ctx, (size_t)n));
-    GPL_TRY(cnt.get(ctx, (size_t)n));
-    GPL_TRY(off.get(ctx, (size_t)n + 2));
-    GPL_TRY(pip_query(ctx, idx, points->xy, points->validity, n, ids.p, cnt.p, ctx->stream));
-    GPL_TRY((exclusive_scan<int32_t, int64_t>(ctx, cnt.p, n, off.p, off.p + n + 1)));
-    int64_t total = 0;
-    GPL_CUDA(cudaMemcpyAsync(&total, off.p + n + 1, sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
-    GPL_CUDA(cudaStreamSynchronize(ctx->stream));
-    if (total == 0) return GPL_OK;
-    void *pl = nullptr, *pr = nullptr;
-    GPL_TRY(ctx->alloc(sizeof(uint64_t) * (size_t)total, &pl));
-    res->lhs = (uint64_t *)pl;
-    GPL_TRY(ctx->alloc(sizeof(uint64_t) * (size_t)total, &pr));
-    res->rhs = (uint64_t *)pr;
-    res->n = total;
-    k_pip_query<1><<<query_grid(n), kQueryThreads, 0, ctx->stream>>>(view_of(idx), reinterpret_cast<const double2 *>(points->xy), points->validity, n,
-                                                                nullptr, nullptr, off.p, res->lhs, res->rhs, 0, nullptr, nullptr, 0);
-    ctx->launches++;
-    GPL_CUDA(cudaGetLastError());
+    GPL_TRY(contains_pairs(ctx, idx, points->xy, points->validity, n, [&](int64_t total, uint64_t **pl, uint64_t **pr) -> int {
+        if (total == 0) return GPL_OK;
+        void *l = nullptr, *r = nullptr;
+        GPL_TRY(ctx->alloc(sizeof(uint64_t) * (size_t)total, &l));
+        res->lhs = (uint64_t *)l;
+        GPL_TRY(ctx->alloc(sizeof(uint64_t) * (size_t)total, &r));
+        res->rhs = (uint64_t *)r;
+        res->n = total;
+        *pl = res->lhs, *pr = res->rhs;
+        return GPL_OK;
+    }));
     GPL_CUDA(cudaStreamSynchronize(ctx->stream));
     return GPL_OK;
 }
@@ -2493,14 +2357,7 @@ extern "C" int gpl_join_histogram(gpl_ctx *ctx, const int32_t *first_id, int64_t
     GPL_REQUIRE(mem == GPL_DEVICE, GPL_ERR_UNSUPPORTED, "gpl_join_histogram: device buffers only");
     GPL_CUDA(cudaSetDevice(ctx->device));
     if (n_points == 0) return GPL_OK;
-    const bool use_smem = n_polygons <= kHistSmemBins;
-    const size_t dyn = use_smem ? sizeof(unsigned int) * (size_t)n_polygons : 0;
-    if (dyn > 48 * 1024) GPL_CUDA(cudaFuncSetAttribute(k_histogram, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn));
-    const int per_sm = use_smem ? (int)std::max<size_t>(1, std::min<size_t>(4, (200 * 1024) / std::max<size_t>(dyn, 1))) : 4;
-    const int grid = (int)std::max<int64_t>(1, std::min<int64_t>(ceil_div(n_points, 2048), (int64_t)kSMs * per_sm));
-    k_histogram<<<grid, 512, dyn, ctx->stream>>>(first_id, n_points, reinterpret_cast<unsigned long long *>(counts), n_polygons,
-                                                 use_smem ? 1 : 0);
-    ctx->launches++;
+    GPL_TRY(launch_histogram(ctx, first_id, n_points, reinterpret_cast<unsigned long long *>(counts), n_polygons, ctx->stream));
     GPL_CUDA(cudaGetLastError());
     return GPL_OK;
 }

@@ -532,7 +532,7 @@ class PipIndex:
                                              C.c_void_p(count_ptr) if count_ptr else None, GPL_DEVICE))
 
     def query_device_counts(self, points_ptr: int, n: int, first_ptr: int, counts_ptr: int) -> None:
-        """join + per-polygon hit counts (u64 column, accumulated) in one pass; all buffers in HBM"""
+        """join + per-polygon hit counts (u64 column, accumulated; a histogram of the id column); all buffers in HBM"""
         check(self.ctx.lib.gpl_contains_join_counts(self.ctx._h, self._h, C.c_void_p(points_ptr), n, C.c_void_p(first_ptr),
                                                     C.c_void_p(counts_ptr), GPL_DEVICE))
 

@@ -259,8 +259,9 @@ int gpl_pip_index_phases(gpl_ctx *ctx, const gpl_pip_index *idx, double *out12);
  * containing rows.  points: xy interleaved, n points, in `mem`. */
 int gpl_contains_join(gpl_ctx *ctx, const gpl_pip_index *idx, const double *points_xy, int64_t n_points,
                       int32_t *first_id, int32_t *count, int mem);
-/* the join and the per-polygon hit counts of config 4 in ONE pass over the points: counts[n polygon rows] (u64) +=
- * number of points whose first containing row is that polygon (what gpl_join_histogram computes from first_id). */
+/* the join and the per-polygon hit counts of config 4: the join (first_id as gpl_contains_join), then a histogram of the
+ * id column, both on the context stream: counts[n polygon rows] (u64) += number of points whose first containing row is
+ * that polygon (what gpl_join_histogram computes from first_id). */
 int gpl_contains_join_counts(gpl_ctx *ctx, const gpl_pip_index *idx, const double *points_xy, int64_t n_points,
                              int32_t *first_id, uint64_t *counts, int mem);
 /* same with the points given as a POINT gpl_array (null points -> -1) */

@@ -53,6 +53,16 @@ def test_product_never_imports_the_oracle():
                     assert "libgeo_oracle" not in code, (f, line)
 
 
+def test_library_reads_no_environment():
+    """the library's behaviour is a function of its inputs: no kernel variant or tuning value is chosen by an environment
+    variable (another build is compared by loading it through GEOPOLARS_B200_LIB instead)"""
+    csrc = os.path.join(ROOT, "geopolars_b200", "csrc")
+    sources = [f for f in os.listdir(csrc) if f.endswith((".cu", ".cuh", ".cpp", ".h")) or f == "Makefile"]
+    assert "k_pip.cu" in sources
+    for f in sources:
+        assert "getenv" not in open(os.path.join(csrc, f), errors="replace").read(), f
+
+
 def test_geoarrow_container_and_row_sharding():
     sq = [(0, 0), (1, 0), (1, 1), (0, 1), (0, 0)]
     mp = GeoArrowArray.from_shapes(GeometryType.MULTIPOLYGON, [[[sq], [sq, sq]], [], [[sq]], None])

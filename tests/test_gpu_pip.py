@@ -294,12 +294,13 @@ def test_reference_golden_envelope_queries_gpu(ctx, og, conv):
                               og.envelope_query(conv(mixed), (-1.0, -1.0, 16.0, 16.0), mode))
 
 
-def test_join_counts_fused_histogram(ctx, og, conv):
-    """gpl_contains_join_counts: ids + per-polygon hit counts in one pass (bins in shared memory up to 12288 polygon rows,
-    the id-column histogram beyond); boundary points (deferred to the exact kernel) must be counted exactly once"""
+def test_join_counts(ctx, og, conv):
+    """gpl_contains_join_counts: ids + per-polygon hit counts, a histogram of the id column after the join (bins in shared
+    memory up to 49152 polygon rows, global atomics beyond); boundary points (deferred to the exact kernel) must be counted
+    exactly once"""
     from geopolars_b200.engine import PipIndex
 
-    for m, grid in ((400, 20), (16_900, 130)):
+    for m, grid in ((400, 20), (16_900, 130), (50_000, 224)):
         xy, ro, go = synth.star_polygons(m, grid)
         polys = GeoArrowArray.polygons(xy, ro, go)
         pts = np.concatenate([synth.uniform_points(300_000, scale=grid * 10.0), xy[:2000], 0.5 * (xy[:2000] + xy[1:2001])])

@@ -1,6 +1,5 @@
 """Round-2 PIP experiments on one B200: build time, query time, raster census for the config-2 workload.
-Knobs are read by the library at load time (environment): GPL_PIP_RASTER_LOG2, GPL_PIP_RASTER_MCELLS,
-GPL_PIP_SLOTS_X100, GPL_PIP_LEGACY, GPL_PIP_STREAM_CTAS_PER_SM, GPL_L2_PIN.  One JSON line per run.
+One JSON line per run.
 
   python tools/exp_pip2.py [--points N] [--polys M --grid G] [--reps R] [--tag TAG]
 """
@@ -73,7 +72,6 @@ with torch.cuda.stream(st):
     fg = stats["fine_cells_per_axis"]
     line = {
         "tag": args.tag, "points": n, "polys": args.polys,
-        "env": {k: v for k, v in os.environ.items() if k.startswith("GPL_")},
         "build_ms_min": min(builds), "build_ms_mean": sum(builds) / len(builds),
         "query_ms_min": min(q), "query_ms_mean": sum(q) / len(q),
         "read_GBps": 16.0 * n / (min(q) * 1e-3) / 1e9,
